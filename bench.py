@@ -9,6 +9,7 @@ ImageNet shape); they are parity cases first and secondary bench lines.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the UNMODIFIED reference (oracle/_ref) on the host CPU cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + what the last timed step computed
 
 One "step" = forward + mean cross-entropy + backward (+ the bucketed NCCL gradient all-reduce of the
 data-parallel ranks, overlapped with backward inside the captured graph) + fused SGD update, through the
@@ -27,6 +28,15 @@ public API of pytorch_ddp_resnet_b200 (GraphedTrainStep).
               if oracle/_ref is absent) timed on the box's host cores on a bounded sample.
 `gpu_reference`: the unmodified reference modules on the SAME GPU through torch + cuDNN: bf16 autocast and the
               reference's literal default (fp16 autocast + GradScaler), batch 128 — the bar to beat.
+
+--dump-outputs DIR (rank 0): after the --steps timed steps, what the last of them handed back: its metrics
+(loss.npy, top1_err.npy, top5_err.npy) and the model state it left (state.<state_dict key>.npy: parameters and
+BatchNorm buffers), float32 (integer buffers float64). Model init, batches and dropout seeds are fixed, and the
+run uses the deterministic mode (B200_DETERMINISTIC=1: fixed-order reductions), so two runs with the same
+arguments write the same arrays and two builds can be compared array for array. The default kernels reduce
+with fp32 atomics: every step differs from run to run in the last bits and training amplifies that (35
+WRN-28-10 steps at lr 0.1: losses 0.62 and 0.59). The numbers of such a run are those of the deterministic mode
+(WRN-28-10, batch 128, one B200 at a 1000 W power limit: 5.21 instead of 4.73 ms/step); time without the flag.
 """
 import argparse
 import json
@@ -368,6 +378,33 @@ def ncu_record():
     return None
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 18   # elements kept of a larger tensor (46.7 MB in all for the largest config, wrn50-imagenet)
+
+
+def dump_outputs(out_dir, metrics, model):
+    """Writes the metrics of a step and the model state after it as <out_dir>/<name>.npy. A tensor of more than
+    DUMP_SAMPLE elements is reduced to a fixed, seeded sample of its flattened elements (logical order, so the
+    memory layout of a build does not move the sample); other tensors keep their shape."""
+    import numpy as np
+    import torch
+    arrays = dict(metrics)
+    arrays.update({"state." + k: v for k, v in model.state_dict().items()})
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.float() if t.is_floating_point() else t.double()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        arrays[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES >> 20} MB limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -437,7 +474,7 @@ def run_ours(args):
             m["loss"].backward()
             opt.step()
             opt.zero_grad(set_to_none=True)
-            return m["loss"]
+            return m
     else:
         # public API: whole-step CUDA graph (pytorch_ddp_resnet_b200.utils.graph_util.GraphedTrainStep)
         from pytorch_ddp_resnet_b200.utils.graph_util import GraphedTrainStep
@@ -453,7 +490,7 @@ def run_ours(args):
         launches_per_step = graphed.launches_per_step
 
         def step(x, y):
-            return graphed(x, y)["loss"]
+            return graphed(x, y)
 
     # ---- device-resident run ---------------------------------------------------------------------
     for i in range(args.warmup):
@@ -461,9 +498,16 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
         time.sleep(0.2)
+    last = {}
+
+    def resident_step(i):
+        last["metrics"] = step(xs_dev[i % nbuf], ys_dev[i % nbuf])
+
     l0 = _lib.launch_count()
-    total_ms = timed(args.steps, lambda i: step(xs_dev[i % nbuf], ys_dev[i % nbuf]), mark=True)
+    total_ms = timed(args.steps, resident_step, mark=True)
     launches = _lib.launch_count() - l0
+    if args.dump_outputs and rank == 0:   # before later steps overwrite the graph's output buffers
+        dump_outputs(args.dump_outputs, last["metrics"], model)
     if launches_per_step is not None:  # replays do not pass through the C ABI: kernels captured per step
         launches = launches_per_step * args.steps
     ms_per_step = total_ms / args.steps
@@ -487,7 +531,7 @@ def run_ours(args):
             y = ys_host[i % nbuf].to(device, non_blocking=True)
         else:  # GraphedTrainStep copies the pinned host batch into its static device buffers
             x, y = xs_host[i % nbuf], ys_host[i % nbuf]
-        loss = step(x, y)
+        loss = step(x, y)["loss"]
         loss_host[i % nbuf].copy_(loss.detach().float(), non_blocking=True)
 
     for i in range(min(3, args.warmup)):
@@ -525,6 +569,7 @@ def run_ours(args):
         "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
         "config": {"workload": cfg["workload"], "name": cfg["name"], "global_batch": B * world,
+                   "deterministic": ops.is_deterministic(),
                    "parallelism": f"dp{world}",
                    "l2": "per-step working set (GBs of saved activations) is far larger than the 126 MB L2; "
                          "4 rotating input batches"},
@@ -610,7 +655,16 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--eager", action="store_true", help="launch every kernel from the host (no CUDA graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the metrics and model state of the last timed step to DIR/<name>.npy; runs the "
+                         "deterministic mode so that runs with the same arguments write the same arrays")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this implementation's timed step computed (--impl ours)")
+    if args.dump_outputs:
+        os.environ["B200_DETERMINISTIC"] = "1"   # read when run_ours imports the package
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         run_reference(args)

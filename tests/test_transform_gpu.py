@@ -56,14 +56,14 @@ def test_kernel_bit_exact_vs_oracle_cifar_shape_batch128(pad_type, whiten):
     assert torch.equal(ob.permute(0, 3, 1, 2), ref.bfloat16())
 
 
-def test_device_loader_feeds_the_model():
+def test_device_loader_feeds_the_model(tmp_path):
     """DeviceDataLoader: one launch per batch, draws made on the device, batches that ResNet.forward takes as
     they are; an epoch visits every sample of the rank's shard once."""
     from pytorch_ddp_resnet_b200.architectures.resnet import ResNet
     from pytorch_ddp_resnet_b200.utils import data_util as D
     aug = {"ToTensorTransform": {}, "StandardizeWhiteningTransform": {}, "FlipTransform": {"p": 0.5},
            "PaddingTransform": {"pad_size": 4, "pad_type": "mirror"}, "RandomCropTransform": {"crop_size": 32}}
-    ds = D.get_datasets("SyntheticCIFAR10", "/tmp", aug, {"ToTensorTransform": {}, "StandardizeWhiteningTransform": {}},
+    ds = D.get_datasets("SyntheticCIFAR10", str(tmp_path), aug, {"ToTensorTransform": {}, "StandardizeWhiteningTransform": {}},
                         synthetic_train_size=256, synthetic_test_size=64)
     sm = D.get_samplers(0, 1, ds["dataset_train"], ds["dataset_test"])
     dl = D.get_dataloaders(64, 1, 1, ds["dataset_train"], ds["dataset_test"], **sm)

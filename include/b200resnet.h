@@ -293,6 +293,24 @@ int b200_sgd_step(float* const* params, const float* const* grads, float* const*
                   const float* inv_scale, const float* found_inf, const float* lr_ptr,
                   b200_stream_t stream);
 
+/* ---- optimizer (torch.optim.Adam / AdamW via get_optimizer('Adam' | 'AdamW', ...)) ---------------------------
+ * One launch for `n` tensors; torch's _single_tensor_adam per element, with t = *steps[i] + 1:
+ * g = grad (* inv_scale); decoupled ? p *= 1 - lr*wd : g += wd * p (only when wd != 0);
+ * m = m + (1-beta1)*(g - m); v = beta2*v + (1-beta2)*g*g; amsgrad: vmax = max(vmax, v), used for v below;
+ * p -= (lr / (1 - beta1^t)) * m / (sqrt(v) / sqrt(1 - beta2^t) + eps), the bias corrections in fp64.
+ * steps: device array of n pointers to fp32 step counters (torch's fused / capturable state['step']); the launch
+ * advances each by one, so a captured graph does at every replay. If found_inf != NULL and *found_inf != 0
+ * nothing is written: not parameters, not moments, not steps (GradScaler contract). lr_ptr (device fp32 scalar,
+ * may be NULL) overrides lr. max_exp_avg_sqs may be NULL unless amsgrad. tickets: n device uint32 counters,
+ * zero on entry and left zero on exit; launches that may run concurrently need separate tickets.
+ * params/grads/exp_avgs/exp_avg_sqs/max_exp_avg_sqs/steps: device arrays of n device pointers; sizes: device
+ * array of n element counts; max_size: the largest of them. 28 B of HBM traffic per element (36 B with amsgrad). */
+int b200_adam_step(float* const* params, const float* const* grads, float* const* exp_avgs,
+                   float* const* exp_avg_sqs, float* const* max_exp_avg_sqs, float* const* steps,
+                   const int64_t* sizes, int n, int64_t max_size, double lr, double beta1, double beta2,
+                   double eps, double weight_decay, int decoupled, int amsgrad, const float* inv_scale,
+                   const float* found_inf, const float* lr_ptr, unsigned* tickets, b200_stream_t stream);
+
 /* *counter += 1 on the device (one launch): the per-step tick of the dropout seed offset. */
 int b200_tick(uint64_t* counter, b200_stream_t stream);
 

@@ -7,7 +7,7 @@ host-side logic (spec parsing, state_dict layout, configs) can be tested without
 """
 import ctypes
 import os
-from ctypes import c_char_p, c_float, c_int, c_int64, c_longlong, c_size_t, c_uint64, c_void_p
+from ctypes import c_char_p, c_double, c_float, c_int, c_int64, c_longlong, c_size_t, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libb200resnet.so")
@@ -60,6 +60,7 @@ SIGNATURES = {
     "b200_ce_topk": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, _P]),
     "b200_sgd_step": (c_int, [_P, _P, _P, _P, c_int, c_int64, c_float, c_float, c_float, c_float,
                               c_int, c_int, _P, _P, _P, _P]),
+    "b200_adam_step": (c_int, [_P] * 7 + [c_int, c_int64] + [c_double] * 5 + [c_int, c_int, _P, _P, _P, _P, _P]),
     "b200_tick": (c_int, [_P, _P]),
     "b200_conv2d_tf32_supported": (c_int, [c_int] + _CONV_DIMS),
     "b200_conv2d_tf32_workspace_bytes": (c_size_t, _CONV_DIMS),

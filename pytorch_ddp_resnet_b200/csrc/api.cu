@@ -2050,6 +2050,26 @@ extern "C" int b200_sgd_step(float* const* params, const float* const* grads, fl
   return 0;
 }
 
+extern "C" int b200_adam_step(float* const* params, const float* const* grads, float* const* exp_avgs,
+                              float* const* exp_avg_sqs, float* const* max_exp_avg_sqs, float* const* steps,
+                              const int64_t* sizes, int n, int64_t max_size, double lr, double beta1,
+                              double beta2, double eps, double weight_decay, int decoupled, int amsgrad,
+                              const float* inv_scale, const float* found_inf, const float* lr_ptr,
+                              unsigned* tickets, b200_stream_t stream) {
+  B200_REQUIRE(params && grads && exp_avgs && exp_avg_sqs && steps && sizes && tickets && n > 0 && max_size >= 0,
+               "adam_step: bad arguments");
+  B200_REQUIRE(!amsgrad || max_exp_avg_sqs, "adam_step: amsgrad needs max_exp_avg_sqs");
+  B200_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0,
+               "adam_step: betas must lie in [0, 1) and eps must be >= 0 (got %g, %g, %g)", beta1, beta2, eps);
+  B200_REQUIRE(n <= 65535, "adam_step: %d tensors in one launch (at most 65535)", n);
+  AdamArgs a{params, grads, exp_avgs, exp_avg_sqs, amsgrad ? max_exp_avg_sqs : nullptr, steps, sizes, tickets,
+             lr, beta1, beta2, eps, weight_decay, decoupled, amsgrad, inv_scale, found_inf, lr_ptr};
+  dim3 grid((unsigned)std::max<int64_t>(1, (max_size + ADAM_CHUNK - 1) / ADAM_CHUNK), n);
+  launch_k(adam_step_kernel, grid, ADAM_THREADS, 0, as_stream(stream), a);
+  B200_LAUNCH_CHECK("adam_step_kernel");
+  return 0;
+}
+
 extern "C" int b200_tick(uint64_t* counter, b200_stream_t stream) {
   B200_REQUIRE(counter, "tick: null pointer");
   launch_k(tick_kernel, 1, 1, 0, as_stream(stream), counter);

@@ -684,6 +684,43 @@ def sgd_step(ptr_table: torch.Tensor, n: int, max_size: int, lr, momentum, dampe
               int(bool(first_step)), _p(inv_scale), _p(found_inf), _p(lr_dev), _stream())
 
 
+_adam_tickets = {}
+
+
+def adam_tickets(device: torch.device, n: int = 0) -> torch.Tensor:
+    """Zero-filled uint32 ticket counters of b200_adam_step (zero on entry, zero again on exit), at least n of
+    them. Keyed like bn_accumulators: one buffer per (device, stream), and one that every capturing stream of
+    the device shares, created together with the first eager buffer so that no fill kernel is recorded into a
+    graph. A capture cannot allocate it: step the optimizer once eagerly before capturing."""
+    capturing = torch.cuda.is_current_stream_capturing()
+    key = (device.index, "capture" if capturing else _stream())
+    t = _adam_tickets.get(key)
+    if t is None or t.numel() < n:
+        if capturing:
+            raise _lib.B200Error("adam_step: ticket counters must be allocated before CUDA-graph capture "
+                                 "(step the optimizer once eagerly first)")
+        t = torch.zeros(max(1024, n), dtype=torch.int32, device=device)
+        _adam_tickets[key] = t
+        cap = _adam_tickets.get((device.index, "capture"))
+        if cap is None or cap.numel() < n:
+            _adam_tickets[(device.index, "capture")] = torch.zeros_like(t)
+    return t
+
+
+def adam_step(ptr_table: torch.Tensor, n: int, max_size: int, lr, beta1, beta2, eps, weight_decay, decoupled,
+              amsgrad, inv_scale=None, found_inf=None, lr_dev=None):
+    """ptr_table: int64 CUDA tensor [7, n] = rows of param, grad, exp_avg, exp_avg_sq, max_exp_avg_sq (unused
+    without amsgrad) and step pointers, then sizes. One launch; it advances every step counter by one."""
+    assert ptr_table.dtype == torch.int64 and ptr_table.is_cuda and ptr_table.shape == (7, n)
+    _lib.require_device(ptr_table.device.index or 0)
+    tickets = adam_tickets(ptr_table.device, n)
+    base = ptr_table.data_ptr()
+    row = n * 8
+    _lib.call("b200_adam_step", *(base + r * row for r in range(7)), n, max_size, float(lr), float(beta1),
+              float(beta2), float(eps), float(weight_decay), int(bool(decoupled)), int(bool(amsgrad)),
+              _p(inv_scale), _p(found_inf), _p(lr_dev), tickets.data_ptr(), _stream())
+
+
 # --------------------------------------------------------------------------------------------------
 # input pipeline
 # --------------------------------------------------------------------------------------------------

@@ -272,7 +272,7 @@ __device__ __forceinline__ uint32_t nonzero_bits8(const uint4& w) {
 // The mask byte comes from the packed OUTPUT when a ReLU is fused (y != 0 exactly where the unit was active and
 // kept): ~16 integer operations per 8 elements instead of a compare + select + merge per element and gate —
 // ncu (round 2) had this kernel at 55 % issue-slot use cold, i.e. issue-bound once the data streams warm.
-// DROP: 0 = no dropout, 1 = dropout, 2 = dropout whose keep bits ARE the mask (no fused ReLU to read it off).
+// DROP: 0 = no dropout, 1 = dropout, 2 = dropout that keeps its keep bits: they ARE the mask when no ReLU is fused.
 template <int U, int MINB, bool SKIP, int DROP>
 __global__ void __launch_bounds__(EW_THREADS, MINB) bn_act_fwd_kernel(const BnActFwdArgs a) {
   const int C = a.C;
@@ -348,7 +348,9 @@ __global__ void __launch_bounds__(EW_THREADS, MINB) bn_act_fwd_kernel(const BnAc
       Vec8 o;
       o.from_float(f);
       if (a.mask_out) {
-        if (DROP != 2 && a.relu) bits = nonzero_bits8(o.raw);
+        // with a fused ReLU the packed output is non-zero exactly where the unit was active AND kept, for every
+        // DROP (the skip route runs DROP == 2 with or without a ReLU); the keep bits alone are the mask without it
+        if (a.relu) bits = nonzero_bits8(o.raw);
         a.mask_out[v] = (uint8_t)bits;
       }
       stg_stream(a.y + v * 8, o.raw);

@@ -75,29 +75,32 @@ def assert_elementwise(out, ref64, mag64, rounding, acc=2.0 ** -14, addends=(), 
     return worst, worst_acc
 
 
-def poisoned(shape, dtype, guard_bytes=4096, device="cuda"):
+def poisoned(shape, dtype, guard_bytes=4096, device="cuda", byte=POISON_BYTE):
     """A tensor of `shape` whose bytes are all 0xFF (NaN), inside a buffer with `guard_bytes` of 0xFF before and
-    after it. The view starts 1024-byte aligned (TMA boxes need 16 B, the epilogues' 256-bit stores 32 B)."""
+    after it. The view starts 1024-byte aligned (TMA boxes need 16 B, the epilogues' 256-bit stores 32 B).
+    byte: another fill for integer outputs, which have no NaN (run them with 0x00 and with 0xFF)."""
     esize = torch.empty((), dtype=dtype).element_size()
     nbytes = esize
     for s in shape:
         nbytes *= s
-    buf = torch.full((guard_bytes + nbytes + guard_bytes + 1024,), POISON_BYTE, dtype=torch.uint8, device=device)
+    buf = torch.full((guard_bytes + nbytes + guard_bytes + 1024,), byte, dtype=torch.uint8, device=device)
     lo = guard_bytes + (-(buf.data_ptr() + guard_bytes)) % 1024
     view = buf[lo:lo + nbytes].view(dtype).view(shape)
     assert view.data_ptr() % 1024 == 0
     view._poison = (buf, lo, lo + nbytes, guard_bytes)
+    view._poison_byte = byte
     return view
 
 
 def check_poisoned(view, label=""):
-    """After a call: both guards of a poisoned() tensor still hold 0xFF bit for bit, and the view holds no NaN (every
-    element was written)."""
+    """After a call: both guards of a poisoned() tensor still hold their fill bit for bit, and the view holds no NaN
+    (every element was written; an integer view cannot show that: compare it exactly under both fills)."""
     buf, lo, hi, guard = view._poison
+    byte = getattr(view, "_poison_byte", POISON_BYTE)
     before = buf[lo - guard:lo]
     after = buf[hi:hi + guard]
     for name, g in (("before", before), ("after", after)):
-        bad = (g != POISON_BYTE).nonzero()
+        bad = (g != byte).nonzero()
         if bad.numel():
             first = int(bad[0].item())
             off = first - guard if name == "before" else first
@@ -163,3 +166,55 @@ def kernels_launched(fn):
             continue
         names.add(normalize_kernel_name(e.name))
     return res, sorted(names)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# the dropout RNG of csrc/common.cuh (rng_draw4, effective_seed) in numpy uint64 arithmetic, and the keep mask that
+# the element-wise BN kernels derive from it
+# ---------------------------------------------------------------------------------------------------------------
+_M32 = 0xFFFFFFFF
+
+
+def rng_draw4(seed, idx):
+    """(x, y) uint32 words of rng_draw4(seed, idx) for an array of counters idx."""
+    import numpy as np
+    idx = np.asarray(idx, dtype=np.uint64)
+    seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    c0 = idx & np.uint64(_M32)
+    c1 = (idx >> np.uint64(32)) ^ np.uint64(seed >> 32)
+    key = seed & _M32
+    for _ in range(4):
+        p = c0 * np.uint64(0xD256D193)                   # < 2^64: c0 < 2^32
+        c0 = (p >> np.uint64(32)) ^ np.uint64(key) ^ c1
+        c1 = p & np.uint64(_M32)
+        key = (key + 0x9E3779B9) & _M32
+    return c0.astype(np.uint32), c1.astype(np.uint32)
+
+
+def effective_seed(seed, offset):
+    """The seed a launch draws with: the host seed plus the device step counter (None: no counter)."""
+    if offset is None:
+        return int(seed) & 0xFFFFFFFFFFFFFFFF
+    return (int(seed) + (int(offset) & 0xFFFFFFFFFFFFFFFF) * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
+
+
+def drop_threshold(p):
+    """api.cu drop_threshold of the fp32 probability: an element is dropped when its 16-bit uniform is below it."""
+    import numpy as np
+    if p <= 0:
+        return 0
+    return min(65535, int(float(np.float32(p)) * 65536.0 + 0.5))
+
+
+def dropout_keep(rows, C, p, seed, offset):
+    """bool [rows, C]: element (r, c) reads half-word c % 4 of draw 2 * (r * C/8 + c/8) + (c % 8) / 4 and is
+    kept when that value is >= drop_threshold(p)."""
+    import numpy as np
+    r = np.arange(rows, dtype=np.uint64)[:, None]
+    c = np.arange(C, dtype=np.uint64)[None, :]
+    draw = np.uint64(2) * (r * np.uint64(C // 8) + c // np.uint64(8)) + (c % np.uint64(8)) // np.uint64(4)
+    x, y = rng_draw4(effective_seed(seed, offset), draw)
+    h = (c % np.uint64(4)).astype(np.uint32)
+    word = np.where(h < 2, x, y)
+    u = np.where(h % 2 == 0, word & np.uint32(0xFFFF), word >> np.uint32(16))
+    return u >= drop_threshold(p)
